@@ -11,6 +11,8 @@ tests/golden/make_rpng_sim_cases.py from the host simulator with seeds 0). Other
 
 Prints ONE JSON line (rank 0). `value` = updates/s with inputs resident in HBM (CUDA events on the engine's stream, L2
 flushed between steps); `e2e` = updates/s through the C-ABI call with host buffers (H2D/D2H inside the timed call).
+`--dump-outputs DIR` also writes the last timed step's results (per-feature status / points / chi², dx, posterior P) as
+DIR/<name>.npy; the inputs are fixed (captured cases, seed-0 synthetic batches), so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -204,36 +206,34 @@ def run_reference(args, rank):
     if w.mode != "msckf":
         print(json.dumps({"impl": "reference", "unavailable": "config 5 is a kernel microbenchmark; the reference arm runs the update configs"}))
         return
-    budget_steps = args.steps
-    # bounded sample: at most ~150 s of CPU work
-    t_probe = time.perf_counter()
-    ups0, r, _ = cpu_updates(w, 1, warm=0)
-    t_one = time.perf_counter() - t_probe
-    budget_steps = int(max(3, min(args.steps, 150.0 / max(t_one, 1e-3))))
-    old = pin_to_one_core()
+    K = args.steps
     from oracle import ovo_py
+    ovo_py.build()
+    old = pin_to_one_core()
     try:
         for _ in range(min(args.warmup, 1)):
             ovo_py.msckf_update(w.frame, w.feats, w.opts, w.P, dumps=False)
         t0 = time.perf_counter()
-        for _ in range(budget_steps):
+        for _ in range(K):
             r = ovo_py.msckf_update(w.frame, w.feats, w.opts, w.P, dumps=False)
         dt = time.perf_counter() - t0
     finally:
         unpin(old)
-    ups = budget_steps / dt
+    ups = K / dt
     line = {
-        "impl": "reference", "metric": "msckf_updates_per_sec", "value": ups, "unit": "updates/s", "n_gpus": args.gpus, "steps": budget_steps,
-        "warmup": args.warmup, "ms_per_step": 1e3 * dt / budget_steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+        "impl": "reference", "metric": "msckf_updates_per_sec", "value": ups, "unit": "updates/s", "n_gpus": args.gpus, "steps": K,
+        "warmup": args.warmup, "ms_per_step": 1e3 * dt / K, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
         "dtype": "f64", "data": w.data, "feats_per_sec": ups * w.n_feats,
         "config": {"workload": w.name, "features_in": int(w.n_feats), "features_used": int(r["stats"].n_feats_used), "rows_stacked": int(r["stats"].rows_stacked),
                    "cols_stacked": int(r["stats"].cols_stacked), "state_dim": int(w.P.shape[0])},
         "cpu_baseline": {"value": ups, "unit": "updates/s", "cores": 1, "kind": "port",
-                         "sample": f"{budget_steps} full updates of the {w.n_feats}-feature batch, one pinned thread (the reference update is single-threaded)"},
+                         "sample": f"{K} full updates of the {w.n_feats}-feature batch, one pinned thread (the reference update is single-threaded)"},
         "e2e": {"value": ups, "unit": "updates/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "features_used": int(r["stats"].n_feats_used), "rows_stacked": int(r["stats"].rows_stacked), "cols_stacked": int(r["stats"].cols_stacked),
         "stage_s": {k: float(v) for k, v in zip(["triangulate", "create_system", "compress", "update"], r["times"])},
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, update_outputs(r["out"], r["dx"], r["P"]))
     print(json.dumps(line), flush=True)
 
 
@@ -258,6 +258,40 @@ def emit(line: dict):
         os.close(_SAVED_STDOUT)
         _SAVED_STDOUT = None
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def update_outputs(out, dx, P) -> dict:
+    """The arrays an MSCKF update hands its caller: the per-feature results, the state correction and the posterior covariance.
+    The C ABI leaves NaN where a rejected feature never got a value (no point after a failed triangulation, no chi² before the
+    gate); its status says so, and 0 stands there instead. A non-finite value of a feature the update used is an error."""
+    from open_vins_b200 import capi
+    used = out.status == capi.FEAT_OK
+    arrays = dict(status=out.status, anchor_cam=out.anchor_cam, anchor_clone=out.anchor_clone, dx=dx, P=P)
+    for k in ("p_FinA", "p_FinG", "chi2"):
+        a = getattr(out, k)
+        bad = ~np.isfinite(a)
+        if (bad.reshape(len(a), -1).any(axis=1) & used).any():
+            raise SystemExit(f"bench.py: --dump-outputs: non-finite {k} of a feature the update used")
+        arrays[k] = np.where(bad, 0.0, a)
+    return arrays
+
+
+def dump_outputs(path: str, arrays: dict):
+    """--dump-outputs: DIR/<name>.npy per array, all float64 (status codes and indices are exact in it) and finite, so that two
+    builds run with the same arguments can be compared output for output."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    bad = [k for k, a in arrays.items() if not np.isfinite(a).all()]
+    if bad:
+        raise SystemExit(f"bench.py: --dump-outputs: non-finite values in {', '.join(bad)}")
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES >> 20} MiB limit")
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------- rooflines
@@ -380,6 +414,9 @@ def bench_update(args, w: Workload, local_rank=0, dist=None, rank=0, world=1):
     ms, stage_sum = eng.msckf_replay(W + K, flush_l2=True)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    # what a caller receives from the last timed step: the per-feature results and dx of the last C-ABI call, and the
+    # posterior covariance the last device-resident replay left on the GPU (same prior and inputs as that call)
+    outputs = update_outputs(out, dx, eng.cov_get()) if args.dump_outputs else None
     ms = ms[W:]
     t_dev = float(ms.sum()) * 1e-3
     stage_ms = stage_sum / float(W + K)
@@ -387,7 +424,8 @@ def bench_update(args, w: Workload, local_rank=0, dist=None, rank=0, world=1):
         tt = torch.tensor([t_e2e, t_dev], dtype=torch.float64, device=torch.device("cuda", local_rank))
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         t_e2e, t_dev = float(tt[0]), float(tt[1])
-    return dict(eng=eng, K=K, W=W, t_e2e=t_e2e, t_dev=t_dev, stage_ms=stage_ms, stats=stats, out=out, cnt=cnt, clocks=clocks, ms=ms)
+    return dict(eng=eng, K=K, W=W, t_e2e=t_e2e, t_dev=t_dev, stage_ms=stage_ms, stats=stats, out=out, cnt=cnt, clocks=clocks, ms=ms,
+                outputs=outputs)
 
 
 def bench_dense(args, w: Workload, local_rank=0):
@@ -396,7 +434,7 @@ def bench_dense(args, w: Workload, local_rank=0):
     import torch
     from open_vins_b200 import capi
     eng = capi.Engine(max_state=512, max_feats=64, max_meas=4096, max_rows=8192, device=local_rank)
-    K, W = max(5, min(args.steps, 50)), args.warmup
+    K, W = args.steps, args.warmup
     n = w.H.shape[1]
     for _ in range(W):
         eng.cov_set(w.P)
@@ -405,8 +443,9 @@ def bench_dense(args, w: Workload, local_rank=0):
     t0 = time.perf_counter()
     for _ in range(K):
         eng.cov_set(w.P)
-        eng.ekf_update([0], [n], w.H, w.res, sigma2=1.0)
+        _, dx = eng.ekf_update([0], [n], w.H, w.res, sigma2=1.0)
     dt = (time.perf_counter() - t0) / K
+    outputs = dict(dx=dx, P=eng.cov_get()) if args.dump_outputs else None
     eng.set_profile(True)
     sums, prof = [], None
     for _ in range(5):
@@ -416,7 +455,7 @@ def bench_dense(args, w: Workload, local_rank=0):
         sums.append(sum(us for _, us in prof))
     eng.set_profile(False)
     eng.close()
-    return dt, K, W, prof, float(np.median(sums)) * 1e-6
+    return dt, K, W, prof, float(np.median(sums)) * 1e-6, outputs
 
 
 def main():
@@ -431,7 +470,11 @@ def main():
                     help="measurement compression: cholqr2 (default, csrc/k_cholqr.cu), tsqr (Householder), gram (one-pass normal equations)")
     ap.add_argument("--features", type=int, default=None, help="synthetic batch with this many features instead of the config's captured case")
     ap.add_argument("--no-sweep", action="store_true", help="N>1: skip the 4096-feature sharded sweep point")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned to its caller as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -456,7 +499,7 @@ def main():
 
     if w.mode == "dense":
         if rank == 0:
-            dt, K, W, prof, t_kernels = bench_dense(args, w, local_rank)
+            dt, K, W, prof, t_kernels, outputs = bench_dense(args, w, local_rank)
             m, n = w.H.shape
             flops = 2.0 * m * n * n - (2.0 / 3.0) * n**3 + 4.0 * m * n + 2.0 * n * n * n + 2 * n**3 / 3.0 + 3.0 * n**3
             ktab = {}
@@ -498,6 +541,8 @@ def main():
                     unpin(old)
                 line["cpu_baseline"] = {"value": 1.0 / float(np.median(ts)), "unit": "updates/s", "cores": 1, "kind": "port",
                                         "sample": f"3 full 8000 x 500 compress + EKFUpdate runs of the oracle (median, {sum(ts):.1f} s), one pinned thread"}
+            if outputs is not None:
+                dump_outputs(args.dump_outputs, outputs)
             emit(line)
         if world > 1:
             dist.barrier()
@@ -507,6 +552,8 @@ def main():
     F = w.n_feats
     rows_total = multigpu.stacked_rows(w.feats.meas_off)
     replicated = world > 1 and rows_total < multigpu.REPLICATE_BELOW_ROWS
+    if args.dump_outputs and world > 1 and not replicated:
+        raise SystemExit("bench.py: --dump-outputs covers the single-GPU and replicated updates, not the sharded one")
     line = None
     if world == 1 or replicated:
         r = bench_update(args, w, local_rank, dist if world > 1 else None, rank, world)
@@ -601,6 +648,8 @@ def main():
                                     "stage_s": {k: float(v) for k, v in zip(["triangulate", "create_system", "compress", "update"], rr["times"])},
                                     "context": cpu_context(w, rr)}
             line["speedup_e2e_vs_cpu_port"] = line["e2e"]["value"] / ups
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         emit(line)
     if world > 1:
         dist.barrier()
